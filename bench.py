@@ -2,7 +2,7 @@
 """bench.py -- contigs/sec of the vamb hot path (VAE train + encode + medoid clustering).
 
 Contract (one JSON line on rank 0):
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--scaling strong|weak]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--scaling strong|weak] [--dump-outputs DIR]
 
 Workload: BASELINE.json configs[1] -- 1,000,000 planted contigs x (103 TNF + 50 abundance samples), `vamb bin
 default` settings (VAE 512-512-32, 300 epochs, batch 256 doubling at epochs 25/75/150/225, then
@@ -48,6 +48,7 @@ import torch  # noqa: E402
 
 METRIC = "contigs/sec (VAE train + cluster) at N=1M, S=50"
 BATCHSTEPS = [25, 75, 150, 225]
+DUMP_ROWS = 1 << 18  # --dump-outputs writes 160 bytes per sampled contig at 32 latent dims: 40 MB at most
 
 
 def parse_args():
@@ -67,7 +68,15 @@ def parse_args():
     ap.add_argument("--time-budget", type=float, default=780.0,
                     help="wall-clock budget (s): optional legs (e2e, cpu_baseline) are skipped, and say so, when the run "
                          "would exceed it")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy: the latent and the clustering of a "
+                         f"fixed, seeded sample of at most {DUMP_ROWS} contigs (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 def schedule(n: int, nepochs: int, batch0: int = 256):
@@ -223,10 +232,12 @@ def epoch_slices(nepochs: int, k: int):
     return [(nepochs * i) // k for i in range(k + 1)]
 
 
-def run_pass(ctx: Ctx, dl, lengths_cluster, nepochs, k_steps, resident: bool, max_clusters=None, batchsteps=None):
+def run_pass(ctx: Ctx, dl, lengths_cluster, nepochs, k_steps, resident: bool, max_clusters=None, batchsteps=None,
+             keep_clusters=False):
     """One pass of the hot path in `k_steps` event-timed steps.  resident=True: the dataset is bound to the device
     before the clock starts, training is driven epoch by epoch and the latent stays in HBM between encode and
-    clustering; resident=False: the public API end to end (trainmodel / encode -> numpy / ClusterGenerator(numpy))."""
+    clustering; resident=False: the public API end to end (trainmodel / encode -> numpy / ClusterGenerator(numpy)).
+    keep_clusters=True also returns the clusters themselves (for --dump-outputs)."""
     import vamb_b200.cluster as vc
     import vamb_b200.encode as ve
     from vamb_b200 import parallel as par
@@ -242,6 +253,7 @@ def run_pass(ctx: Ctx, dl, lengths_cluster, nepochs, k_steps, resident: bool, ma
     ctx.barrier()
     step_ms, phases = [], {"train": 0.0, "encode": 0.0, "cluster": 0.0}
     n_clusters = n_members = probes = evals = 0
+    clusters = [] if keep_clusters else None
     cluster_timing = {}
     latent_dev = None
     t_wall0 = time.perf_counter()
@@ -284,6 +296,8 @@ def run_pass(ctx: Ctx, dl, lengths_cluster, nepochs, k_steps, resident: bool, ma
                 for c in gen:
                     n_clusters += 1
                     n_members += len(c.members)
+                    if clusters is not None:
+                        clusters.append(c)
                     if max_clusters and n_clusters >= max_clusters:
                         break
                 probes, evals = gen._n_probes, gen._n_evals
@@ -312,7 +326,37 @@ def run_pass(ctx: Ctx, dl, lengths_cluster, nepochs, k_steps, resident: bool, ma
             "n_clusters": n_clusters, "n_clustered": n_members, "probes": probes, "evals": evals,
             "train_steps": sum(s * e for _, s, e in sched), "launches": launches,
             "final_loss": vae._last_epoch_losses[0], "vae": vae, "latent_dev": latent_dev,
-            "cluster_timing": cluster_timing}
+            "cluster_timing": cluster_timing, "clusters": clusters}
+
+
+def dump_outputs(out_dir, latent_dev, clusters, seed):
+    """What the last timed step hands a caller -- the encoder's latent and the clusters -- for a fixed sample of
+    contigs (the same rows for the same --contigs and --seed), so two builds can be compared output for output:
+      rows.npy            (R,) float64     contig indices of the sample, ascending
+      latent.npy          (R, L) float32   their latent rows, as encode returns them
+      cluster_index.npy   (R,) float64     emission order of the cluster each contig fell into
+      cluster_medoid.npy  (R,) float64     that cluster's medoid (a contig index)
+      cluster_radius.npy  (R,) float64     that cluster's radius, -1 where it has none (a loner)
+    R = min(contigs, DUMP_ROWS)."""
+    n = latent_dev.shape[0]
+    rows = np.sort(np.random.default_rng(seed).choice(n, min(n, DUMP_ROWS), replace=False))
+    index = np.full(n, -1, dtype=np.int64)
+    medoid = np.empty(len(clusters), dtype=np.int64)
+    radius = np.empty(len(clusters), dtype=np.float64)
+    for k, c in enumerate(clusters):
+        index[np.asarray(c.members)] = k
+        medoid[k] = c.medoid
+        radius[k] = -1.0 if c.radius is None else c.radius  # a radius is a distance, >= 0; every output is finite
+    assert (index[rows] >= 0).all(), "a sampled contig is in no cluster"
+    k = index[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"rows": rows.astype(np.float64),
+              "latent": latent_dev[torch.from_numpy(rows).to(latent_dev.device)].cpu().numpy(),
+              "cluster_index": k.astype(np.float64), "cluster_medoid": medoid[k].astype(np.float64),
+              "cluster_radius": radius[k]}
+    for name, x in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), x)
+    return sorted(arrays)
 
 
 def vae_roofline(vae, n, nepochs):
@@ -521,8 +565,12 @@ def main():
     sampler = ClockSampler(ctx.local_rank)
     sampler.start()
     log(f"timed pass: {args.steps} steps (dataset resident in HBM)")
-    res = run_pass(ctx, dl, lens_cluster, args.nepochs, max(1, args.steps), resident=True)
+    res = run_pass(ctx, dl, lens_cluster, args.nepochs, args.steps, resident=True,
+                   keep_clusters=args.dump_outputs is not None)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        names = dump_outputs(args.dump_outputs, res["latent_dev"], res["clusters"], args.seed)
+        log(f"outputs of the last timed step: {', '.join(names)} in {args.dump_outputs}")
     t_pass = ctx.max_over_ranks(res["t_event"])
     value = n_total / t_pass
     log(f"  {t_pass:.2f}s: train {res['phases']['train']:.2f} encode {res['phases']['encode']:.2f} cluster "

@@ -22,4 +22,8 @@ vae_oracle.py      torch-CPU fp32 restatement of vamb/encode.py (forward, loss,
 csrc/oracle_kernels.c   the C inner loops of cluster_oracle (gcc, -ffp-contract=off).
 make_golden.py     runs the real reference (via ref_loader) and writes
                    tests/golden/*.npz; committed together with its outputs.
+numerics.py        pins torch's CPU arithmetic so that bit-exact fixtures hold on
+                   any x86-64 host (called by tests/conftest.py and the writers).
+make_golden_reference.py   the same for the reference's dataloader, VAE steps,
+                   trainmodel losses and clusters of its own test fixture.
 """

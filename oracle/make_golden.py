@@ -69,8 +69,9 @@ def make_cluster_goldens(ref):
 
 
 def main():
-    from oracle import ref_loader
+    from oracle import numerics, ref_loader
 
+    numerics.pin()
     os.makedirs(GOLDEN, exist_ok=True)
     ref = ref_loader.load()
     make_cluster_goldens(ref)

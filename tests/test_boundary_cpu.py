@@ -2,6 +2,8 @@
 symbol, and argument validation raises the reference's exceptions before any GPU work."""
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -42,13 +44,17 @@ def test_probe_header_layout_matches_binding():
 
 
 def test_no_cpu_fallback():
-    import torch
-    from vamb_b200 import _lib
-
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(_lib.VkError):
-        _lib.require_device()
+    """With no CUDA device visible, require_device() raises instead of running on the CPU.  A child process with
+    CUDA_VISIBLE_DEVICES="" sees no device, so this also runs on a machine that has one."""
+    code = ("from vamb_b200 import _lib\n"
+            "try:\n"
+            "    _lib.require_device()\n"
+            "except _lib.VkError:\n"
+            "    print('refused')\n")
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=env, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.strip() == "refused"
 
 
 class TestClusterBadParams:

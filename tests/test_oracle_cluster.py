@@ -2,16 +2,18 @@
 
  * golden fixtures (tests/golden/cluster_*.npz) were produced by the UNMODIFIED reference
    (oracle/make_golden.py); the oracle must reproduce every cluster exactly;
- * when /root/reference is present (build container) the oracle is also compared with the
-   live reference on the reference's own test fixture (test/test_cluster.py:11-13);
+ * the oracle also reproduces the reference's clusters of the reference's own test fixture
+   (test/test_cluster.py:11-13), stored by oracle/make_golden_reference.py;
  * restated known-answer pieces: histogram edges, smoothing kernel, in-place mask array.
 """
+import os
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import cluster_oracle as co
-from oracle import ref_loader
+from oracle import make_golden_reference as mgr
 from tests import _util
 
 
@@ -25,16 +27,11 @@ def test_oracle_matches_reference_golden(name):
     assert len(allm) == len(lat) and set(allm.tolist()) == set(range(len(lat)))
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present (GPU box)")
 def test_oracle_matches_live_reference_on_reference_fixture():
-    ref = ref_loader.load()
-    rng = np.random.RandomState(5)
-    data = rng.random((1024, 40)).astype(np.float32)
-    lens = rng.randint(500, 1000, size=1024)
-    order = np.argsort(lens)[::-1]
-    rc = list(ref.cluster.ClusterGenerator(data, lens))
-    oc = list(co.OracleClusterGenerator(data, lens, order=order))
-    _util.assert_clusters_equal(oc, rc)
+    g = np.load(os.path.join(_util.GOLDEN, "ref_cluster_fixture.npz"))
+    data, lens = mgr.cluster_fixture()
+    oc = list(co.OracleClusterGenerator(data, lens, order=g["order"]))
+    _util.assert_clusters_equal_golden(oc, g)
 
 
 def test_histogram_edges_are_torch_linspace():

@@ -1,13 +1,13 @@
 """CPU suite: the torch-fp32 VAE oracle is PINNED -- it reproduces the reference-made golden fixtures bit for bit
-(tests/golden/vae_*.npz, written by oracle/make_golden_vae.py from the unmodified reference), and, where the
-reference tree is present (build container), the live reference itself.  Also pins oracle/normalize.py."""
+(tests/golden/vae_*.npz, written by oracle/make_golden_vae.py, and tests/golden/ref_*.npz, written by
+oracle/make_golden_reference.py, both from the unmodified reference).  Also pins oracle/normalize.py."""
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import ref_loader
+from oracle import make_golden_reference as mgr
 from oracle import vae_oracle as vo
 from oracle.make_golden_vae import VAE_CASES, vae_inputs
 
@@ -63,83 +63,61 @@ def test_normalize_restatement_matches_the_product_dataloader():
         assert np.array_equal(x, y.numpy())
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree only exists in the build container")
 def test_normalize_restatement_matches_the_live_reference():
+    """oracle/normalize.py == the reference's make_dataloader tensors (tests/golden/ref_dataloader_*.npz)."""
     from oracle import normalize as onorm
-    from oracle import synth
 
-    ref = ref_loader.load()
-    ab, tnf, lens = synth.make_contigs(2000, 3, seed=5)
-    want = ref.encode.make_dataloader(ab.copy(), tnf.copy(), lens).dataset.tensors
-    for x, y in zip(onorm.normalize(ab, tnf, lens), want):
-        assert np.array_equal(x, y.numpy())
+    name = "synth_2000x3"
+    g = np.load(os.path.join(GOLDEN, f"ref_dataloader_{name}.npz"))
+    ab, tnf, lens = mgr.dataloader_inputs(name)
+    for k, x in zip("dtaw", onorm.normalize(ab, tnf, lens)):
+        mgr.assert_digest_and_sample(g, k, x)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree only exists in the build container")
 def test_vae_oracle_equals_live_reference_over_training_steps():
     """Under the same ``torch.manual_seed`` stream the oracle and the unmodified reference stay bit-identical
-    (losses, every parameter and buffer, encode) over 6 optimiser steps."""
-    from oracle import dadapt
+    (losses, every parameter and buffer, encode) over 6 optimiser steps (tests/golden/ref_vae_steps.npz)."""
+    from oracle import normalize as onorm
 
-    ref = ref_loader.load()
-    S, n, batch, seed = 5, 400, 64, 11
+    c = mgr.VAE_STEPS
+    g = np.load(os.path.join(GOLDEN, "ref_vae_steps.npz"))
+    S, n, batch, seed = c["S"], c["n"], c["batch"], c["seed"]
     rpkm, tnfs, lens = vae_inputs(S, n, seed)
-    dl = ref.encode.make_dataloader(rpkm.copy(), tnfs.copy(), lens, batchsize=batch)
-    d, t, a, w = dl.dataset.tensors
-    vae = ref.encode.VAE(S, nhiddens=[64, 48], nlatent=12, seed=seed)
-    o = vo.OracleVAE(S, nhiddens=[64, 48], nlatent=12, seed=seed)
-    opt = dadapt.DAdaptAdam(vae.parameters(), decouple=True)
-    vae.train()
+    d, t, a, w = (torch.from_numpy(x) for x in onorm.normalize(rpkm, tnfs, lens))
+    o = vo.OracleVAE(S, nhiddens=c["nhiddens"], nlatent=c["nlatent"], seed=seed)
     rng = np.random.default_rng(seed)
-    for step in range(6):
+    for step in range(c["nsteps"]):
         idx = torch.from_numpy(rng.choice(n, size=batch, replace=False).astype(np.int64))
-        torch.manual_seed(2000 + step)
-        opt.zero_grad()
-        do, to, ao, mu = vae(d[idx], t[idx], a[idx])
-        L = vae.calc_loss(d[idx], do, t[idx], to, a[idx], ao, mu, w[idx])
-        L[0].backward()
-        opt.step()
-        torch.manual_seed(2000 + step)
+        torch.manual_seed(c["torch_seed0"] + step)
         lo, _, _ = o.train_step(d[idx], t[idx], a[idx], w[idx])
-        assert [float(x.detach()) for x in L] == lo
-    for k, v in vae.state_dict().items():
-        assert torch.equal(v, o.state[k]), k
-    vae.eval()
-    assert np.array_equal(vae.encode(dl), o.encode(d, t, a, batch=batch)[0])
+        assert lo == list(g["losses"][step]), (step, lo, g["losses"][step])
+    state_keys = sorted(k[len("state."):] for k in g.files if k.startswith("state."))
+    assert state_keys == sorted(o.state)
+    for k in state_keys:
+        assert mgr.sha256(o.state[k].numpy()) == str(g[f"state.{k}"]), k  # every parameter and buffer, bit for bit
+    mgr.assert_digest_and_sample(g, "latent", o.encode(d, t, a, batch=batch)[0])
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree only exists in the build container")
 def test_strict_rng_emulation_follows_the_live_reference_trainmodel():
     """``vamb_b200.encode.reference_epoch_noise`` (the strict-RNG parity mode of the CUDA path) consumes torch's global
     generator exactly like the reference's DataLoader + forward pass: driving the (bit-exact) oracle with it reproduces
-    the per-epoch losses that the unmodified ``VAE.trainmodel`` logs, including a batch-size doubling."""
-    import re
-
+    the per-epoch losses that the unmodified ``VAE.trainmodel`` logs, including a batch-size doubling
+    (tests/golden/ref_trainmodel_losses.npz)."""
     pytest.importorskip("vamb_b200._lib")
-    from loguru import logger
 
     import vamb_b200.encode as ve
     from oracle import normalize as onorm
     from oracle import synth
 
-    ref = ref_loader.load()
-    S, n, seed, nepochs, bsteps = 4, 1500, 3, 4, [2]
-    ab, tnf, lens = synth.make_contigs(n, S, seed=8)
-    rows = []
-    pat = re.compile(r"Epoch:\s*(\d+)\s+Loss:\s*(\S+)")
-    logger.enable("vamb")
-    sink = logger.add(lambda m: rows.append(pat.search(str(m))), level="INFO")
-    dl = ref.encode.make_dataloader(ab.copy(), tnf.copy(), lens, batchsize=128)
-    vae = ref.encode.VAE(S, nhiddens=[64, 32], nlatent=8, seed=seed)
-    vae.trainmodel(dl, nepochs=nepochs, batchsteps=bsteps)
-    logger.remove(sink)
-    logger.disable("vamb")
-    want = [float(m.group(2)) for m in rows if m]
+    c = mgr.TRAINMODEL
+    S, n, seed, nepochs, bsteps = c["S"], c["n"], c["seed"], c["nepochs"], c["batchsteps"]
+    ab, tnf, lens = synth.make_contigs(n, S, seed=c["data_seed"])
+    want = np.load(os.path.join(GOLDEN, "ref_trainmodel_losses.npz"))["epoch_loss"].tolist()
     assert len(want) == nepochs
 
     d, t, a, w = (torch.from_numpy(x) for x in onorm.normalize(ab, tnf, lens))
-    o = vo.OracleVAE(S, nhiddens=[64, 32], nlatent=8, seed=seed)  # torch.manual_seed(seed) + the reference's init draws
-    batch, got = 128, []
+    o = vo.OracleVAE(S, nhiddens=c["nhiddens"], nlatent=c["nlatent"], seed=seed)  # torch.manual_seed(seed) + the reference's init draws
+    batch, got = c["batch"], []
     for epoch in range(nepochs):
         if epoch in bsteps:
             batch *= 2
